@@ -2,6 +2,7 @@
 """bench.py -- image-pairs/s of the dense-descriptor training hot path (fwd(A) + fwd(B) + loss + backward) at 640x480.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c5] [--two-calls]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -330,6 +331,24 @@ def gpu_torch_baseline_leg(cfg, H, W, dev):
     return {"workload": "same step as `value` (inputs resident), 3 timed steps after 2 warm-up", "rows": rows}
 
 
+DUMP_SAMPLE = 1 << 21      # elements kept of a larger array: three 8 MB samples + the loss values stay well under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy, float32 (float64 for the loss values).  An array of more than DUMP_SAMPLE
+    elements is replaced by the flattened elements at DUMP_SAMPLE sorted flat indices drawn without replacement by
+    numpy.random.default_rng(0) -- the same indices for the same shape -- so that two builds run with the same arguments
+    can be compared element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def committed_traffic(kernel_class):
     """dram bytes per launch of the dominant kernel class from the committed `ncu --set full` capture, if there is one."""
     p = os.path.join(ROOT, "profiles", "r2_traffic.json")
@@ -388,6 +407,7 @@ def run_ours(args, cfg):
     h2d_bytes = sum(pinned[k].numel() * pinned[k].element_size() for k in keys)
 
     side = [torch.cuda.Stream(device=dev), torch.cuda.Stream(device=dev)] if args.two_streams else None
+    last = {}                 # --dump-outputs: what the latest step handed back to its caller
 
     def forward_loss_backward(d):
         if args.two_streams:      # EXPERIMENT (timing only: shared BN buffers / pack cache / flat gradient are raced)
@@ -408,6 +428,8 @@ def run_ours(args, cfg):
                                       d["matches_a"], d["matches_b"], d["masked_a"], d["masked_b"],
                                       d["background_a"], d["background_b"], blind, blind)
         five[0].backward()
+        if args.dump_outputs:
+            last.update(five=five, descriptors_a=ya, descriptors_b=yb)
         return five[0]
 
     def step(d):
@@ -453,6 +475,14 @@ def run_ours(args, cfg):
 
     with ClockSampler(local_rank) as clk:
         ms_total, launches, loss, host_ms = timed_steps(False)
+    if args.dump_outputs and rank == 0:
+        # the last timed step: its five loss values, both descriptor batches and every parameter gradient (after the
+        # all-reduce), concatenated in named_parameters() order
+        dump_outputs(args.dump_outputs, {
+            "loss": torch.tensor([float(t.detach()) for t in last["five"]], dtype=torch.float64),
+            "descriptors_a": last["descriptors_a"], "descriptors_b": last["descriptors_b"],
+            "param_grads": torch.cat([p.grad.reshape(-1) for _, p in dcn.named_parameters()])})
+        last.clear()
     # ---- timed region 1b: the same K steps again with a CUDA-event pair around every convolution / loss kernel on the launching
     # stream (ddn_profile_*): the per-class kernel durations the roofline block is computed from
     if args.profile_run:      # under ncu: warm-up + the timed steps only, so the launch list is exactly `steps` steps
@@ -643,7 +673,12 @@ def main():
                     help="configs[4] variant: use_l2_pixel_loss_on_masked_non_matches=True (M_pixel=50)")
     ap.add_argument("--profile-run", action="store_true",
                     help="short run for ncu: 1 warm-up + --steps timed steps, no e2e / cpu legs (numbers printed are NOT bench values)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss values, descriptors, parameter "
+                         "gradients; seeded samples of the large arrays) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.pairs_per_gpu is not None:
         cfg["pairs_per_gpu"] = args.pairs_per_gpu

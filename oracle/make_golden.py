@@ -22,11 +22,12 @@ sys.path.insert(0, os.path.join(ROOT, "pytorch-dense-correspondence_b200"))
 from oracle import loss_oracle as LO            # noqa: E402
 from oracle import build_ref                    # noqa: E402
 from oracle import ref_loader                   # noqa: E402
-from oracle.resnet34_8s_oracle import seeded_oracle, process_network_output  # noqa: E402
+from oracle import ref_cases                    # noqa: E402
+from oracle.resnet34_8s_oracle import GOLDEN_CPU_THREADS, seeded_oracle, process_network_output  # noqa: E402
 import synthetic                                # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
-torch.set_num_threads(os.cpu_count())
+torch.set_num_threads(GOLDEN_CPU_THREADS)
 
 
 def bit_equal(a, b, what):
@@ -137,8 +138,158 @@ def train_step_case(name, D, B, H, W, Nm, Nn, seed):
     print("wrote", name, "five", out["five"])
 
 
+def assert_same(x, y, what):
+    """Bit-equal results (tensors, numbers, strings, None, and tuples / lists / dicts of them)."""
+    if isinstance(x, torch.Tensor):
+        assert isinstance(y, torch.Tensor) and x.dtype == y.dtype, what
+        bit_equal(x, y, what)
+    elif isinstance(x, (tuple, list)):
+        assert isinstance(y, (tuple, list)) and len(x) == len(y), what
+        for i, (a, b) in enumerate(zip(x, y)):
+            assert_same(a, b, "%s[%d]" % (what, i))
+    elif isinstance(x, dict):
+        assert sorted(x) == sorted(y), what
+        for k in x:
+            assert_same(x[k], y[k], "%s/%s" % (what, k))
+    else:
+        assert x == y, (what, x, y)
+
+
+def ref_loss_cases():
+    """Every PixelwiseContrastiveLoss method and every loss_composer branch (oracle/ref_cases.py), run on the executed
+    reference; the torch restatement must agree bit-for-bit."""
+    ref = build_ref.load()
+    H, W, D, P = 12, 20, 5, 240
+    gen = torch.Generator().manual_seed(3)
+    A = 0.3 * torch.randn(1, P, D, generator=gen); B = 0.3 * torch.randn(1, P, D, generator=gen)
+    ma = torch.randint(0, P, (7,), generator=gen); mb = torch.randint(0, P, (7,), generator=gen)
+    inp = dict(H=H, W=W, A=A, B=B, ma=ma, mb=mb, na=ma.repeat_interleave(4), nb=torch.randint(0, P, (28,), generator=gen))
+    out = ref_cases.loss_methods(ref.pcl.PixelwiseContrastiveLoss, inp)
+    assert_same(ref_cases.loss_methods(LO.TorchPixelwiseContrastiveLoss, inp), out, "loss methods")
+    torch.save({"inputs": inp, "outputs": out}, os.path.join(GOLD, "ref_loss_methods.pt"))
+
+    H, W, D, P = 10, 16, 3, 160
+    gen = torch.Generator().manual_seed(9)
+    A = 0.3 * torch.randn(1, D, H, W, generator=gen); B = 0.3 * torch.randn(1, D, H, W, generator=gen)
+    ma = torch.randint(0, P, (6,), generator=gen); mb = torch.randint(0, P, (6,), generator=gen)
+    idx = dict(matches_a=ma, matches_b=mb, masked_a=ma.repeat_interleave(3), masked_b=torch.randint(0, P, (18,), generator=gen),
+               background_a=ma.repeat_interleave(2), background_b=torch.randint(0, P, (12,), generator=gen),
+               blind_a=torch.randint(0, P, (9,), generator=gen), blind_b=torch.randint(0, P, (9,), generator=gen))
+    inp = dict(A=A, B=B, idx=idx)
+    SD = ref.dataset.SpartanDataset
+    out = ref_cases.composer_branches(ref.pcl.PixelwiseContrastiveLoss, ref.composer.get_loss, SD.empty_tensor, inp)
+    assert_same(ref_cases.composer_branches(LO.TorchPixelwiseContrastiveLoss, LO.get_loss, LO.empty_tensor, inp), out, "composer")
+    out["empty_tensor"] = SD.empty_tensor()
+    T = ref.dataset.SpartanDatasetDataType
+    out["data_types"] = {k: getattr(T, k) for k in dir(T) if k.isupper()}
+    torch.save({"inputs": inp, "outputs": out}, os.path.join(GOLD, "ref_composer_branches.pt"))
+    print("wrote ref_loss_methods, ref_composer_branches")
+
+
+def _with_rand(fn, fake):
+    """fn() with torch.rand replaced by fake (the reference samplers draw their uniforms from it)."""
+    real = torch.rand
+    torch.rand = fake
+    try:
+        return fn()
+    finally:
+        torch.rand = real
+
+
+def ref_non_match_sampler_case():
+    """create_non_correspondences draws torch.rand(n) (mask branch) or torch.rand(2, n) (no mask), then two more draws for the
+    no-op perturbation; the restatement takes the uniforms as arguments -- feed both the same numbers."""
+    ref = build_ref.load()
+    H, W, k = 30, 40, 5
+    gen = torch.Generator().manual_seed(4)
+    ma = torch.randint(0, H * W, (11,), generator=gen)
+    uv_a = (ma % W, ma // W)
+    uv_b = ((ma % W).float(), (ma // W).float())
+    n = len(ma) * k
+    ru, rv = torch.rand(n, generator=gen), torch.rand(n, generator=gen)
+    mask = torch.zeros(H, W); mask[5:20, 8:30] = 1.0
+    masks, outs = [mask, None, torch.zeros(H, W)], []
+    SD = ref.dataset.SpartanDataset
+    for m in masks:
+        calls = []
+
+        def fake_rand(*shape):
+            calls.append(shape)
+            if len(calls) == 1:
+                return ru.clone() if shape == (n,) else torch.stack((ru, rv)).clone()
+            return torch.zeros(*shape)
+        uv_b_non = _with_rand(lambda: ref.finder.create_non_correspondences(uv_b, (H, W), num_non_matches_per_match=k, img_b_mask=m),
+                              fake_rand)
+        uv_a_long, uv_b_long = SD.create_non_matches(None, uv_a, uv_b_non, k)
+        na_r = SD.flatten_uv_tensor(uv_a_long, W).squeeze(1); nb_r = SD.flatten_uv_tensor(uv_b_long, W).squeeze(1)
+        assert_same(list(LO.create_non_correspondences_flat(ma, (H, W), k, m, ru, rv)), [na_r, nb_r], "sampler")
+        outs.append((na_r, nb_r))
+    torch.save({"inputs": dict(H=H, W=W, k=k, matches_a=ma, rand_u=ru, rand_v=rv, masks=masks), "outputs": outs},
+               os.path.join(GOLD, "ref_non_match_sampler.pt"))
+    print("wrote ref_non_match_sampler", [len(o[1]) for o in outs])
+
+
+def ref_reprojection_case():
+    """batch_find_pixel_correspondences on a rendered tilted plane with no-return pixels and an occluder."""
+    ref = build_ref.load()
+    H, W, n = 120, 160, 900
+    K = np.array([[133.4, 0, 79.8], [0, 133.7, 59.1], [0, 0, 1.0]])
+
+    def pose(rx, ry, t):
+        cx, sx, cy, sy = np.cos(rx), np.sin(rx), np.cos(ry), np.sin(ry)
+        Rx = np.array([[1, 0, 0], [0, cx, -sx], [0, sx, cx]]); Ry = np.array([[cy, 0, sy], [0, 1, 0], [-sy, 0, cy]])
+        T = np.eye(4); T[:3, :3] = Ry.dot(Rx); T[:3, 3] = t
+        return T
+    pa, pb = pose(0.01, -0.02, [0, 0, 0]), pose(-0.04, 0.1, [0.15, -0.03, 0.04])
+    nrm, d0 = np.array([-0.1, 0.05, 1.0]), 1.2
+
+    def render(T):
+        us, vs = np.meshgrid(np.arange(W), np.arange(H))
+        rays = np.linalg.inv(K).dot(np.stack([us.ravel(), vs.ravel(), np.ones(H * W)]))
+        s = (d0 - nrm.dot(T[:3, 3])) / nrm.dot(T[:3, :3].dot(rays))
+        return (s * 1000.0).reshape(H, W)
+    da = np.round(render(pa)).astype(np.uint16); db = np.round(render(pb)).astype(np.uint16)
+    da[10:30, 20:50] = 0                                               # no-return pixels (depth 0) are pruned
+    db[60:80, 100:130] = 300                                           # an occluder in front of the plane in image b
+    mask = np.zeros((H, W), dtype=np.float32); mask[5:110, 10:150] = 1.0
+    ru = torch.rand(n, generator=torch.Generator().manual_seed(8))
+    # the reference first draws (and discards) rand(2, n) for unmasked candidates, then rand(n) for the masked sample
+    uv_a, uv_b = _with_rand(lambda: ref.finder.batch_find_pixel_correspondences(da, pa, db, pb, num_attempts=n, img_a_mask=mask, K=K),
+                            lambda *s: ru.clone() if s == (n,) else torch.zeros(*s))
+    nz = torch.nonzero(torch.from_numpy(mask).view(-1))
+    cand = torch.index_select(nz, 0, torch.floor(ru * len(nz)).long()).squeeze(1)
+    uv_a_o, uv_b_o = LO.batch_find_pixel_correspondences(da, pa, db, pb, cand, K)
+    assert_same(list(uv_a_o) + list(uv_b_o), list(uv_a) + list(uv_b), "reprojection")
+    inp = {k: torch.from_numpy(v.astype(np.int32) if v.dtype == np.uint16 else v)
+           for k, v in dict(depth_a=da, pose_a=pa, depth_b=db, pose_b=pb, K=K, mask_a=mask).items()}
+    inp["rand"] = ru
+    torch.save({"inputs": inp, "outputs": list(uv_a) + list(uv_b)}, os.path.join(GOLD, "ref_reprojection.pt"))
+    print("wrote ref_reprojection", len(uv_a[0]), "of", n)
+
+
+def ref_backbone_modules_case():
+    """The reference modules themselves at D = 8: parameter names, the dilation bookkeeping, train- and eval-mode outputs."""
+    D = 8
+    oracle = seeded_oracle(D=D, seed=0)
+    ref = ref_loader.reference_resnet34_8s(D, oracle.state_dict())
+    x = torch.randn(1, 3, 40, 56, generator=torch.Generator().manual_seed(2))
+    out = {"x": x.numpy(), "state_dict_keys": np.array(list(ref.state_dict().keys()))}
+    for mode in ("train", "eval"):
+        getattr(ref, mode)(); getattr(oracle, mode)()
+        y = ref(x).detach()
+        bit_equal(y, oracle(x).detach(), "backbone modules " + mode)
+        out["y_" + mode] = y.numpy()
+    r = ref.resnet34_8s
+    for name, v in (("layer3.0.conv1.dilation", r.layer3[0].conv1.dilation), ("layer3.0.conv1.padding", r.layer3[0].conv1.padding),
+                    ("layer4.0.conv1.dilation", r.layer4[0].conv1.dilation), ("layer4.0.downsample.0.stride", r.layer4[0].downsample[0].stride),
+                    ("layer2.0.conv1.stride", r.layer2[0].conv1.stride), ("layer2.0.downsample.0.stride", r.layer2[0].downsample[0].stride)):
+        out["attr:" + name] = np.array(v)
+    np.savez_compressed(os.path.join(GOLD, "ref_backbone_modules_d8.npz"), **out)
+    print("wrote ref_backbone_modules_d8")
+
+
 if __name__ == "__main__":
-    assert ref_loader.reference_available() and build_ref.reference_available(), "needs /root/reference"
+    assert ref_loader.reference_available() and build_ref.reference_available(), "needs the reference checkout"
     build_ref.build()
     os.makedirs(GOLD, exist_ok=True)
     backbone_case("backbone_small_d3", D=3, B=2, H=64, W=96, seed_data=11)
@@ -151,3 +302,7 @@ if __name__ == "__main__":
     loss_case("loss_noscale_d16", 16, 48, 64, 64, 2, 1, 5, {"scale_by_hard_negatives": False, "M_masked": 1.5,
                                                              "M_background": 1.2}, 23)
     train_step_case("train_step_small_d3", D=3, B=2, H=64, W=96, Nm=40, Nn=120, seed=31)
+    ref_loss_cases()
+    ref_non_match_sampler_case()
+    ref_reprojection_case()
+    ref_backbone_modules_case()

@@ -1,6 +1,6 @@
 """CPU: the oracle reproduces the committed golden vectors (which were written from the REAL reference by
-oracle/make_golden.py), the numpy and torch loss restatements agree, and -- when /root/reference is present
-(build container) -- the oracle is re-checked bit-for-bit against the reference modules."""
+oracle/make_golden.py), the numpy and torch loss restatements agree, and the oracle equals the reference modules on the
+inputs stored with their outputs."""
 import os
 
 import numpy as np
@@ -8,8 +8,7 @@ import pytest
 import torch
 
 from oracle import loss_oracle as LO
-from oracle import ref_loader
-from oracle.resnet34_8s_oracle import seeded_oracle, process_network_output
+from oracle.resnet34_8s_oracle import GOLDEN_CPU_THREADS, seeded_oracle, process_network_output
 import pdc_b200
 from pdc_b200 import synthetic
 
@@ -18,8 +17,16 @@ def _load(golden_dir, name):
     return np.load(os.path.join(golden_dir, name + ".npz"))
 
 
+@pytest.fixture
+def golden_threads():
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_CPU_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("name,D,B,H,W", [("backbone_small_d3", 3, 2, 64, 96), ("backbone_small_d16", 16, 1, 48, 64)])
-def test_backbone_oracle_matches_golden(golden_dir, name, D, B, H, W):
+def test_backbone_oracle_matches_golden(golden_dir, golden_threads, name, D, B, H, W):
     g = _load(golden_dir, name)
     net = seeded_oracle(D=D, seed=0)
     x = torch.randn(B, 3, H, W, generator=torch.Generator().manual_seed(int(g["x_seed"])))
@@ -104,7 +111,7 @@ def test_loss_oracle_edge_cases():
         LO.get_loss(pcl, torch.tensor([1]), A, B, one, two, one, two, one, two, one, two)
 
 
-def test_train_step_oracle_matches_golden(golden_dir):
+def test_train_step_oracle_matches_golden(golden_dir, golden_threads):
     g = _load(golden_dir, "train_step_small_d3")
     D, B, H, W = 3, 2, 64, 96
     net = seeded_oracle(D=D, seed=0).train()
@@ -134,22 +141,27 @@ def test_synthetic_structure():
     assert all(torch.equal(d[k], d2[k]) for k in d if d[k] is not None)
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference only exists in the build container")
-def test_oracle_bit_equal_to_reference_modules():
-    D = 8
-    oracle = seeded_oracle(D=D, seed=0)
-    ref = ref_loader.reference_resnet34_8s(D, oracle.state_dict())
-    assert list(ref.state_dict().keys()) == list(oracle.state_dict().keys())
-    assert len(ref.state_dict()) == 218
-    x = torch.randn(1, 3, 40, 56, generator=torch.Generator().manual_seed(2))
+def test_oracle_bit_equal_to_reference_modules(golden_dir, golden_threads):
+    """The reference's own Resnet34_8s (D = 8) was loaded with this oracle's seeded weights by oracle/make_golden.py, which
+    checked bit-equality there and stored the reference's parameter names, dilation bookkeeping and outputs."""
+    g = _load(golden_dir, "ref_backbone_modules_d8")
+    oracle = seeded_oracle(D=8, seed=0)
+    assert list(oracle.state_dict().keys()) == [str(k) for k in g["state_dict_keys"]]
+    assert len(g["state_dict_keys"]) == 218
+    x = torch.tensor(g["x"])
     for mode in ("train", "eval"):
-        getattr(ref, mode)(); getattr(oracle, mode)()
-        assert torch.equal(ref(x), oracle(x)), mode
+        getattr(oracle, mode)()
+        # same torch build -> bit equal; a different CPU/torch build may reorder fp32 sums
+        np.testing.assert_allclose(oracle(x).detach().numpy(), g["y_" + mode], rtol=1e-4, atol=1e-5, err_msg=mode)
     # the dilation bookkeeping the modern torchvision API gets differently (SURVEY.md 3.2)
-    r = ref.resnet34_8s
-    assert r.layer3[0].conv1.dilation == (2, 2) and r.layer3[0].conv1.padding == (2, 2)
-    assert r.layer4[0].conv1.dilation == (4, 4) and r.layer4[0].downsample[0].stride == (1, 1)
-    assert r.layer2[0].conv1.stride == (2, 2) and r.layer2[0].downsample[0].stride == (2, 2)
+    r = oracle.resnet34_8s
+    for name, got, want in (("layer3.0.conv1.dilation", r.layer3[0].conv1.dilation, (2, 2)),
+                            ("layer3.0.conv1.padding", r.layer3[0].conv1.padding, (2, 2)),
+                            ("layer4.0.conv1.dilation", r.layer4[0].conv1.dilation, (4, 4)),
+                            ("layer4.0.downsample.0.stride", r.layer4[0].downsample[0].stride, (1, 1)),
+                            ("layer2.0.conv1.stride", r.layer2[0].conv1.stride, (2, 2)),
+                            ("layer2.0.downsample.0.stride", r.layer2[0].downsample[0].stride, (2, 2))):
+        assert tuple(g["attr:" + name]) == want and tuple(got) == want, name
 
 
 def test_reprojection_oracle_against_ray_cast_ground_truth():
