@@ -445,6 +445,14 @@ static int build_terms_lr(const ddn_loss_term* th, int n_terms, DevTerms* T, int
 }
 static float ac_scale(int in, int out) { return out > 1 ? (float)(in - 1) / (float)(out - 1) : 0.f; }
 
+// The D = 4 / 8 / 16 / 32 kernels read and reduce 16-byte vectors, so their maps must start 16-byte aligned; a cell row is then a
+// multiple of 16 bytes for every D % 4 == 0.  The other D take scalar accesses and accept any float-aligned map -- e.g. the
+// second half of forward_pair's output at D = 3, which starts B * h * w * 12 bytes into the buffer.
+static bool lowres_aligned(int D, const void* a, const void* b, const void* c = nullptr, const void* d = nullptr) {
+  if (D % 4 != 0) return true;
+  return ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c) | reinterpret_cast<uintptr_t>(d)) & 15) == 0;
+}
+
 }  // namespace ddn
 
 using namespace ddn;
@@ -454,6 +462,7 @@ extern "C" int ddn_contrastive_terms_forward_lowres(const float* low_a, const fl
                                                     double* sums, int64_t* counts, void* stream) {
   DDN_TRY(check_common(low_a, low_b, B, (int64_t)H * W, D, W));
   DDN_CHECK_ARG(sums && counts && h >= 1 && w >= 1 && H >= h && W >= w && (int64_t)H * W < (1LL << 31), "bad low-resolution geometry / null outputs");
+  DDN_CHECK_ARG(lowres_aligned(D, low_a, low_b), "low-resolution maps must be 16-byte aligned when D is a multiple of 4");
   const int lpp = (D == 8 || D == 16 || D == 32) ? D / 4 : 1;
   // 4 pairs per lane group; 8 (DDN_LOSS_FWD_ITEMS=8) halves the atomics again but costs occupancy: 17.4 -> 18.7-20.9 us at C3
   static const int items = [] { const char* e = getenv("DDN_LOSS_FWD_ITEMS"); return (e && atoi(e) == 8) ? 8 : 4; }();
@@ -494,8 +503,8 @@ extern "C" int ddn_contrastive_terms_backward_lowres(const float* low_a, const f
                                                      float* dlow_a, float* dlow_b, void* stream) {
   DDN_TRY(check_common(low_a, low_b, B, (int64_t)H * W, D, W));
   DDN_CHECK_ARG(coef && dlow_a && dlow_b && h >= 1 && w >= 1 && H >= h && W >= w && (int64_t)H * W < (1LL << 31), "bad low-resolution geometry / null buffers");
-  DDN_CHECK_ARG(((reinterpret_cast<uintptr_t>(dlow_a) | reinterpret_cast<uintptr_t>(dlow_b) | reinterpret_cast<uintptr_t>(low_a) | reinterpret_cast<uintptr_t>(low_b)) & 15) == 0,
-                "low-resolution maps and their gradients must be 16-byte aligned");
+  DDN_CHECK_ARG(lowres_aligned(D, low_a, low_b, dlow_a, dlow_b),
+                "low-resolution maps and their gradients must be 16-byte aligned when D is a multiple of 4");
   const int lpp = (D == 8 || D == 16 || D == 32) ? D / 4 : 1;
   DevTerms T;
   DDN_TRY(build_terms_lr(terms_host, n_terms, &T, LR_THREADS / lpp));

@@ -11,6 +11,7 @@ import torch
 import pdc_b200
 from pdc_b200 import loss_composer, synthetic, _native as N
 from oracle import loss_oracle as LO
+from oracle import well_conditioned as WC
 from oracle.resnet34_8s_oracle import seeded_oracle, process_network_output
 
 pytestmark = pytest.mark.gpu
@@ -314,49 +315,21 @@ def test_weight_pack_cache_follows_parameter_updates():
 
 
 # ---------------------------------------------------------------------------------------------------- round 2
-def _decisive_relu_biases(net, amp=3.0, on_fraction=0.7, seed=5):
-    """BatchNorm biases set to +-amp (70 % of the channels +amp, 30 % -amp): almost every ReLU input is then several standard
-    deviations away from zero, so the ReLU masks -- both the passing and the blocking kind -- are the SAME in every arithmetic,
-    and the gradient of the whole network becomes a well-conditioned function of its inputs (fp32 vs fp64 CPU oracle: ~3e-6 per
-    tensor instead of ~1e-2 with the default biases, where a handful of mask flips at |pre-activation| ~ 1 ulp dominate)."""
-    g = torch.Generator().manual_seed(seed)
-    with torch.no_grad():
-        for k, p in net.named_parameters():
-            if ("bn" in k or "downsample.1" in k) and k.endswith(".bias"):
-                sign = (torch.rand(p.shape, generator=g) < on_fraction).to(p.dtype) * 2 - 1
-                p.copy_(amp * sign)
-    return net
-
-
-def _well_conditioned_case(precision, mode, D, B, H, W, seed):
-    gen = torch.Generator().manual_seed(seed)
-    x = torch.randn(B, 3, H, W, generator=gen)
-    cot = torch.randn(B, D, H, W, generator=gen)
-    oracle = _decisive_relu_biases(seeded_oracle(D=D, seed=0))
-    if mode == "eval":      # frozen statistics that actually normalise: one pass with momentum 1 copies the batch statistics
-        bns = [m for m in oracle.modules() if isinstance(m, torch.nn.BatchNorm2d)]
-        for m in bns:
-            m.momentum = 1.0
-        oracle.train()
-        with torch.no_grad():
-            oracle(x)
-        for m in bns:
-            m.momentum = 0.1
+def _well_conditioned_case(precision, mode, D, B, H, W, seed, groups=1):
+    """groups=1: one call of the network on B images.  groups=2: forward_pair(A, B) on two batches of B images, gated against
+    two fp64 oracle calls (A then B) with the gradients of both summed."""
+    x, cot, oracle = WC.build(mode, D, B, H, W, seed, groups)
     net, _ = make_net(D, precision, oracle)
-    ref64 = seeded_oracle(D=D, seed=0).double()
-    ref64.load_state_dict({k: v.double() if v.is_floating_point() else v for k, v in oracle.state_dict().items()})
-    for m in (oracle, net, ref64):
-        m.train(mode == "train")
-    y = net(x.to(DEV))
-    y64 = ref64(x.double())
-    assert rel(y, y64.detach()) < (2e-5 if precision == "fp32" else 1e-3)
+    net.train(mode == "train")
+    if groups == 1:
+        y = net(x.to(DEV))
+    else:
+        dcn = pdc_b200.DenseCorrespondenceNetwork(net, D, image_width=W, image_height=H)
+        ya, yb = dcn.forward_pair(x[:B].to(DEV), x[B:].to(DEV))
+        y = torch.cat([ya, yb])
+    y64, g64, big, scale, cert = WC.reference(oracle, mode, x, cot, groups)
+    assert rel(y, y64) < (2e-5 if precision == "fp32" else 1e-3)
     (y * cot.to(DEV)).sum().backward()
-    (y64 * cot.double()).sum().backward()
-    y32 = oracle(x); (y32 * cot).sum().backward()      # the fp32 CPU oracle's own distance from fp64: the conditioning certificate
-    g64 = {k: p.grad for k, p in ref64.named_parameters()}
-    scale = max(float(v.norm()) for v in g64.values())
-    big = [k for k in g64 if float(g64[k].norm()) >= 1e-6 * scale]
-    cert = max(rel(p.grad, g64[k]) for k, p in oracle.named_parameters() if k in big)
     assert cert < 1e-4, "gradients should be well conditioned here (fp32 oracle vs fp64: %.2e)" % cert
     gate = 2e-4 if precision == "fp32" else 1e-3
     if mode == "eval" and precision != "fp32":
@@ -385,6 +358,35 @@ def _well_conditioned_case(precision, mode, D, B, H, W, seed):
     return (not failures), worst, cert, net, oracle, y, cot
 
 
+def _check_well_conditioned_gradients(precision, mode, D, B, H, W, groups=1, seeds=WC.SEEDS):
+    # One construction is not decisive: relu(bn2(.) + identity), where a -3 channel of bn2 meets a positive identity and the sum can
+    # land within the forward error of zero (~1e-7 relative for the fp32 oracle, ~1e-5 for bf16x3: with ~10^6 such elements the
+    # tensor-core path flips one in roughly every second input, the oracle in one of a few hundred).  The ONE flipped mask element
+    # then shows up at the 1e-2 level in every tensor upstream of it -- for that input, in that arithmetic.  A kernel bug does not
+    # depend on the input seed, a flip does: up to six inputs are tried, every one of them has to stay within flip noise (1e-1: observed 1e-2 .. 2.4e-2),
+    # and the tight gate has to be met on at least one (the message lists the inputs that flipped).
+    report = []
+    for seed in seeds:
+        ok_tight, worst, cert, net, oracle, y, cot = _well_conditioned_case(precision, mode, D, B, H, W, seed, groups)
+        report.append((seed, worst))
+        if ok_tight:
+            break
+    assert ok_tight, "tight gate missed on every input seed: %s" % report
+    print("well-conditioned whole-net gradients [%s, %s-mode BN, D=%d, %d x %d image(s) of %dx%d]: worst per-tensor rel err %.2e "
+          "(fp32 CPU oracle vs fp64: %.1e)%s"
+          % (precision, mode, D, groups, B, H, W, worst, cert, "" if len(report) == 1 else "  [mask flips on input seeds %s: %s]" %
+             ([r[0] for r in report[:-1]], ["%.1e" % r[1] for r in report[:-1]])))
+    sd = net.state_dict(); so = oracle.state_dict()
+    if mode == "eval":      # running statistics untouched by an eval-mode forward + backward
+        assert torch.equal(sd["resnet34_8s.bn1.running_mean"].cpu(), so["resnet34_8s.bn1.running_mean"])
+    else:                   # updated once per group, A then B, like the oracle's calls
+        assert rel(sd["resnet34_8s.layer4.2.bn2.running_var"], so["resnet34_8s.layer4.2.bn2.running_var"]) < 1e-4
+        assert rel(sd["resnet34_8s.layer1.0.bn1.running_mean"], so["resnet34_8s.layer1.0.bn1.running_mean"]) < 1e-4
+        assert int(sd["resnet34_8s.bn1.num_batches_tracked"]) == int(so["resnet34_8s.bn1.num_batches_tracked"])
+    with pytest.raises(RuntimeError):          # a second backward through the same graph is refused with a clear message
+        (y * cot.to(DEV)).sum().backward()
+
+
 @pytest.mark.parametrize("precision", PRECISIONS)
 @pytest.mark.parametrize("mode", ["train", "eval"])
 @pytest.mark.parametrize("D,B,H,W", [(3, 2, 64, 96), (8, 1, 120, 160)])
@@ -393,33 +395,49 @@ def test_whole_network_gradients_well_conditioned(precision, mode, D, B, H, W):
     backward with batch statistics, residual adds, max-pool, fc, upsample) gated TIGHTLY per tensor against the oracle in fp64.
     The usual obstacle -- ReLU / max-pool decisions that flip on 1-ulp differences give this randomly initialised network a
     1e-2 gradient noise floor even between PyTorch's own CPU and CUDA runs -- is removed by making the ReLU decisions
-    decisive (see _decisive_relu_biases), NOT by loosening the gate; the fp32 CPU oracle's own distance from fp64 is asserted
+    decisive (see oracle/well_conditioned.py), NOT by loosening the gate; the fp32 CPU oracle's own distance from fp64 is asserted
     as the conditioning certificate (< 1e-4).  train: batch statistics (the training path).  eval: frozen running statistics --
     the reference backpropagates through an eval()-mode network via autograd, here DDN_MODE_EVAL_SAVE."""
     tc_or_skip(precision)
-    # One construction is not decisive: relu(bn2(.) + identity), where a -3 channel of bn2 meets a positive identity and the sum can
-    # land within the forward error of zero (~1e-7 relative for the fp32 oracle, ~1e-5 for bf16x3: with ~10^6 such elements the
-    # tensor-core path flips one in roughly every second input, the oracle in one of a few hundred).  The ONE flipped mask element
-    # then shows up at the 1e-2 level in every tensor upstream of it -- for that input, in that arithmetic.  A kernel bug does not
-    # depend on the input seed, a flip does: up to six inputs are tried, every one of them has to stay within flip noise (1e-1: observed 1e-2 .. 2.4e-2),
-    # and the tight gate has to be met on at least one (the message lists the inputs that flipped).
-    report = []
-    for seed in (77, 78, 79, 80, 81, 82):
-        ok_tight, worst, cert, net, oracle, y, cot = _well_conditioned_case(precision, mode, D, B, H, W, seed)
-        report.append((seed, worst))
-        if ok_tight:
-            break
-    assert ok_tight, "tight gate missed on every input seed: %s" % report
-    print("well-conditioned whole-net gradients [%s, %s-mode BN, D=%d]: worst per-tensor rel err %.2e (fp32 CPU oracle vs fp64: %.1e)%s"
-          % (precision, mode, D, worst, cert, "" if len(report) == 1 else "  [mask flips on input seeds %s: %s]" %
-             ([r[0] for r in report[:-1]], ["%.1e" % r[1] for r in report[:-1]])))
-    sd = net.state_dict(); so = oracle.state_dict()
-    if mode == "eval":      # running statistics untouched by an eval-mode forward + backward
-        assert torch.equal(sd["resnet34_8s.bn1.running_mean"].cpu(), so["resnet34_8s.bn1.running_mean"])
-    else:
-        assert rel(sd["resnet34_8s.layer4.2.bn2.running_var"], so["resnet34_8s.layer4.2.bn2.running_var"]) < 1e-4
-    with pytest.raises(RuntimeError):          # a second backward through the same graph is refused with a clear message
-        (y * cot.to(DEV)).sum().backward()
+    _check_well_conditioned_gradients(precision, mode, D, B, H, W)
+
+
+@pytest.mark.parametrize("precision", PRECISIONS)
+@pytest.mark.parametrize("case", WC.CASES, ids=WC.case_id)
+def test_whole_network_gradients_over_shapes_descriptor_sizes_and_groups(precision, case):
+    """The gate of test_whole_network_gradients_well_conditioned over the matrix of oracle/well_conditioned.py: the layer-1 halo
+    kernels with their BatchNorm epilogues, CTAs and CTA pairs whose sub-tiles belong to different BatchNorm groups
+    (forward_pair), descriptor sizes below and at each fc template size, and the minimum shapes."""
+    tc_or_skip(precision)
+    D, B, groups, H, W, mode, seeds = case
+    _check_well_conditioned_gradients(precision, mode, D, B, H, W, groups, seeds)
+
+
+@pytest.mark.parametrize("precision", PRECISIONS)
+@pytest.mark.parametrize("case", [c for c in WC.CASES if c[5] == "train"], ids=lambda c: WC.case_id(c, with_mode=False))
+def test_inference_forward_over_shapes_descriptor_sizes_and_groups(precision, case):
+    """eval() without gradients runs DDN_MODE_INFER: BatchNorm folded into the conv epilogues (the layer-1 halo kernels'
+    folded epilogue included).  Against the fp64 oracle in eval mode with the frozen statistics of oracle/well_conditioned.py;
+    groups=2 goes through forward_pair, which must then be two independent eval-mode calls."""
+    tc_or_skip(precision)
+    D, B, groups, H, W, _, seeds = case
+    x, _, oracle = WC.build("eval", D, B, H, W, seeds[0], groups)
+    net, _ = make_net(D, precision, oracle)
+    net.eval()
+    ref64 = seeded_oracle(D=D, seed=0).double().eval()
+    ref64.load_state_dict({k: v.double() if v.is_floating_point() else v for k, v in oracle.state_dict().items()})
+    with torch.no_grad():
+        if groups == 1:
+            y = net(x.to(DEV))
+        else:
+            dcn = pdc_b200.DenseCorrespondenceNetwork(net, D, image_width=W, image_height=H)
+            y = torch.cat(dcn.forward_pair(x[:B].to(DEV), x[B:].to(DEV)))
+        y64 = ref64(x.double())
+    assert not y.requires_grad
+    e = rel(y, y64)
+    print("inference forward [%s, %s]: rel err %.2e" % (precision, WC.case_id(case, with_mode=False), e))
+    assert e < (2e-5 if precision == "fp32" else 1e-3)
+    assert torch.equal(net.state_dict()["resnet34_8s.bn1.running_mean"].cpu(), oracle.state_dict()["resnet34_8s.bn1.running_mean"])
 
 
 @pytest.mark.parametrize("precision", PRECISIONS)
@@ -574,3 +592,72 @@ def test_weight_pack_cache_cannot_go_stale():
     y_ref = fresh(x).detach()
     assert rel(y1, y_ref) < 1e-6, "stale packed weights in use"
     assert rel(y1, y0) > 1e-3
+
+
+LOSS_SHAPES = sorted({(D, B, H, W) for D, B, _, H, W, _, _ in WC.CASES})        # (D, images per batch, H, W)
+
+
+def _hard_negative_bounds(A, Bm, ia, ib, margin):
+    """The hard-negative count of a hinge term is exact except for pairs whose fp64 distance lies within 1e-6 of the margin."""
+    d = np.sqrt(((A[ia].astype(np.float64) - Bm[ib].astype(np.float64)) ** 2).sum(1))
+    return int((d < margin - 1e-6).sum()), int((d < margin + 1e-6).sum())
+
+
+@pytest.mark.parametrize("api", ["two_calls", "forward_pair"])
+@pytest.mark.parametrize("D,B,H,W", LOSS_SHAPES)
+def test_fused_loss_step_at_the_shape_matrix(monkeypatch, api, D, B, H, W):
+    """A training step (forward A / B, get_loss with all four terms, backward) at the shapes and descriptor sizes of
+    oracle/well_conditioned.py: the loss fused with the upsample (default) equals the generic gather (DDN_FUSED_UPSAMPLE_LOSS=0)
+    -- five outputs, hard-negative counts, parameter gradients -- and the fused loss equals the float64 restatement
+    LO.np_within_scene_loss evaluated on the network's own descriptors.  Low-resolution maps with h*w odd or not a multiple of 4
+    (40x48: 30 cells, 72x40: 45) put forward_pair's second half at an offset that is not 16-byte aligned."""
+    tc_or_skip("bf16x3")
+    data = synthetic.make_pair_batch(B, H, W, 40, 120, 120, 17, seed=31 + D)
+    d = {k: v.to(DEV) for k, v in data.items()}
+    cfg = dict(LO.DEFAULT_LOSS_CONFIG)
+    outs = {}
+    for fused in ("1", "0"):
+        monkeypatch.setenv("DDN_FUSED_UPSAMPLE_LOSS", fused)
+        dcn = pdc_b200.DenseCorrespondenceNetwork.from_config({"descriptor_dimension": D, "image_width": W, "image_height": H},
+                                                              load_stored_params=False)
+        dcn.fcn.load_state_dict(seeded_oracle(D=D, seed=0).state_dict())
+        dcn.train()
+        pcl = pdc_b200.PixelwiseContrastiveLoss(dcn.image_shape, dict(cfg))
+        pcl.debug = True
+        if api == "forward_pair":
+            a, b = dcn.forward_pair(d["img_a"], d["img_b"])
+        else:
+            a, b = dcn.forward(d["img_a"]), dcn.forward(d["img_b"])
+        pa, pb = dcn.process_network_output(a, B), dcn.process_network_output(b, B)
+        assert pdc_b200.resnet_dilated.lowres_of(pa) is not None and pdc_b200.resnet_dilated.lowres_of(pb) is not None
+        five = loss_composer.get_loss(pcl, torch.zeros(B, dtype=torch.int64), pa, pb, d["matches_a"], d["matches_b"], d["masked_a"],
+                                      d["masked_b"], d["background_a"], d["background_b"], d["blind_a"], d["blind_b"])
+        five[0].backward()
+        outs[fused] = ([float(t) for t in five], pcl.debug_data["num_hard_negatives_device"].cpu(),
+                       {k: p.grad.detach().clone() for k, p in dcn.fcn.named_parameters()}, pa.detach().cpu(), pb.detach().cpu())
+    (f1, c1, g1, pa1, pb1), (f0, c0, g0, _, _) = outs["1"], outs["0"]
+    assert torch.equal(c1, c0)
+    for x, y in zip(f1, f0):
+        assert abs(x - y) <= 2e-6 * max(1.0, abs(y)), (f1, f0)
+    assert rel(g1["resnet34_8s.fc.weight"], g0["resnet34_8s.fc.weight"]) < 1e-4
+    num = sum(float((g1[k].double() - g0[k].double()).norm() ** 2) for k in g0); den = sum(float(g0[k].double().norm() ** 2) for k in g0)
+    assert (num / den) ** 0.5 < 1e-3
+    # the fused loss against float64 on the same descriptors (mean over the pairs of the per-pair loss)
+    five64 = np.zeros(5)
+    counts_equal = True
+    hinge_terms = [("masked_a", "masked_b", cfg["M_masked"]), ("background_a", "background_b", cfg["M_background"]),
+                   ("blind_a", "blind_b", cfg["M_masked"])]
+    for i in range(B):
+        A, Bm = pa1[i].numpy(), pb1[i].numpy()
+        idx = {k: data[k][i].numpy() for k in ("matches_a", "matches_b", "masked_a", "masked_b", "background_a", "background_b",
+                                               "blind_a", "blind_b")}
+        vals, hard = LO.np_within_scene_loss(A, Bm, idx, cfg, W)
+        five64 += np.array(vals) / B
+        for t, (ka, kb, margin) in enumerate(hinge_terms):
+            lo, hi = _hard_negative_bounds(A, Bm, idx[ka], idx[kb], margin)
+            got = int(c1[i, t + 1])
+            assert lo <= got <= hi, (i, ka, got, lo, hi)
+            counts_equal &= got == hard[t]
+    if counts_equal:        # (a count that differs on a pair at the margin changes the scale, not an error of the kernels)
+        for x, y in zip(f1, five64):
+            assert abs(x - y) <= 1e-5 * abs(y) + 1e-12, (f1, list(five64))

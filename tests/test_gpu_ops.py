@@ -387,15 +387,22 @@ def test_device_reprojection_match_finder_vs_restated_reference():
 # ---------------------------------------------------------------------------------------------------- round 2
 @pytest.mark.parametrize("over", [{}, {"scale_by_hard_negatives": False},
                                   {"use_l2_pixel_loss_on_masked_non_matches": True, "use_l2_pixel_loss_on_background_non_matches": True, "M_pixel": 9}])
-def test_ragged_batch_matches_the_reference_loop(over):
+@pytest.mark.parametrize("path", ["generic", "fused"])
+def test_ragged_batch_matches_the_reference_loop(path, over):
     """Real SpartanDataset samples have a different number of matches per pair (num_matching_attempts is only an upper bound,
     dataset/spartan_dataset_masked.py:652-660), so a batch is ragged: rows padded with -1 + per-pair counts.  The fused loss
     must equal the mean over the pairs of the reference's per-pair loss on the un-padded lists (values, all five outputs,
-    gradients)."""
+    gradients).  generic: gathered from full-resolution descriptor images.  fused: the images are bilinear upsamples of
+    low-resolution maps they are tagged with (what Resnet34_8s returns), so the loss runs through csrc/loss_lowres.cu and the
+    gradient w.r.t. the low-resolution maps is compared."""
     H, W, D, B = 24, 32, 4, 3
     P = H * W
     gen = torch.Generator().manual_seed(11)
-    A = 0.3 * torch.randn(B, D, H, W, generator=gen); Bt = 0.3 * torch.randn(B, D, H, W, generator=gen)
+    if path == "generic":
+        A = 0.3 * torch.randn(B, D, H, W, generator=gen); Bt = 0.3 * torch.randn(B, D, H, W, generator=gen)
+    else:
+        lows = [(0.3 * torch.randn(B, D, H // 8, W // 8, generator=gen)).requires_grad_() for _ in range(2)]
+        A, Bt = [F.interpolate(t, size=(H, W), mode="bilinear", align_corners=True) for t in lows]
     n_match, k_m, k_b, n_blind = [41, 7, 23], 3, 2, [5, 0, 9]
     lists = {k: [] for k in ("matches_a", "matches_b", "masked_a", "masked_b", "background_a", "background_b", "blind_a", "blind_b")}
     for b in range(B):
@@ -409,7 +416,7 @@ def test_ragged_batch_matches_the_reference_loop(over):
             lists["blind_a"].append(LO.empty_tensor()); lists["blind_b"].append(LO.empty_tensor())
     cfg = dict(LO.DEFAULT_LOSS_CONFIG); cfg.update(over)
     # reference: per-pair loop over the un-padded lists, mean over pairs
-    Ar = A.clone().requires_grad_(); Br = Bt.clone().requires_grad_()
+    Ar = A.detach().clone().requires_grad_(); Br = Bt.detach().clone().requires_grad_()
     ref = LO.TorchPixelwiseContrastiveLoss([H, W], dict(cfg))
     par, pbr = process_network_output(Ar, B, D, H, W), process_network_output(Br, B, D, H, W)
     outs = [LO.get_within_scene_loss(ref, par[b:b + 1], pbr[b:b + 1], *[lists[k][b] for k in
@@ -417,8 +424,12 @@ def test_ragged_batch_matches_the_reference_loop(over):
     five_r = [sum(o[i].reshape(()) for o in outs) / B for i in range(5)]
     five_r[0].backward()
     # ours: padded [B, n_max] + per-pair counts
-    Ag = A.to(DEV).requires_grad_(); Bg = Bt.to(DEV).requires_grad_()
+    Ag = A.detach().to(DEV).requires_grad_(); Bg = Bt.detach().to(DEV).requires_grad_()
     pag, pbg = process_network_output(Ag, B, D, H, W), process_network_output(Bg, B, D, H, W)
+    if path == "fused":
+        low_g = [nhwc(t.detach()).reshape(B, (H // 8) * (W // 8), D).to(DEV).requires_grad_() for t in lows]
+        from pdc_b200 import resnet_dilated
+        resnet_dilated.attach_lowres(pag, low_g[0], H, W); resnet_dilated.attach_lowres(pbg, low_g[1], H, W)
     pad = {k: loss_composer.pad_index_lists(v, device=DEV) for k, v in lists.items()}
     blind_len = torch.tensor([n if n else 0 for n in n_blind], dtype=torch.int64, device=DEV)
     nv = {"matches": pad["matches_a"][1], "masked": pad["masked_a"][1], "background": pad["background_a"][1], "blind": blind_len}
@@ -429,7 +440,13 @@ def test_ragged_batch_matches_the_reference_loop(over):
     for i in range(5):
         assert abs(float(five[i]) - float(five_r[i])) <= 2e-6 * max(1.0, abs(float(five_r[i]))), (i, float(five[i]), float(five_r[i]))
     five[0].backward()
-    assert rel(Ag.grad, Ar.grad) < 1e-5 and rel(Bg.grad, Br.grad) < 1e-5
+    if path == "generic":
+        assert rel(Ag.grad, Ar.grad) < 1e-5 and rel(Bg.grad, Br.grad) < 1e-5
+    else:                   # the full-resolution images were never differentiated; upsample^T of the reference gradient
+        assert Ag.grad is None and Bg.grad is None
+        A.backward(Ar.grad); Bt.backward(Br.grad)
+        for t_g, t_r in zip(low_g, lows):
+            assert rel(t_g.grad, nhwc(t_r.grad).reshape(B, -1, D)) < 1e-5
 
 
 def test_triplet_loss_matches_the_oracle():
@@ -462,12 +479,25 @@ def test_triplet_loss_matches_the_oracle():
 
 @pytest.mark.parametrize("D,over", [(3, {}), (16, {}), (8, {"use_l2_pixel_loss_on_masked_non_matches": True, "M_pixel": 9,
                                                         "scale_by_hard_negatives": False}),
-                                    (32, {}), (5, {}), (16, {"use_l2_pixel_loss_on_masked_non_matches": True, "M_pixel": 25})])
+                                    (32, {}), (5, {}), (16, {"use_l2_pixel_loss_on_masked_non_matches": True, "M_pixel": 25}),
+                                    (1, {}), (4, {}), (4, {"use_l2_pixel_loss_on_background_non_matches": True, "M_pixel": 9}),
+                                    (12, {}), (24, {})])
 def test_loss_fused_with_the_upsample_equals_the_generic_loss(D, over):
     """csrc/loss_lowres.cu: the loss evaluated through the bilinear upsample (4 low-resolution cells per sampled pixel) must equal
     the loss gathered from the upsampled image -- all five outputs, hard-negative counts -- and its gradient w.r.t. the
-    low-resolution map must equal upsample^T of the generic path's full-resolution gradient."""
-    B, H, W = 2, 64, 96
+    low-resolution map must equal upsample^T of the generic path's full-resolution gradient.  D = 4 is the float4 / red.v4
+    instantiation, 8 / 16 / 32 the channel-quad kernels, every other D the run-time-D scalar kernel."""
+    _check_fused_loss_equals_generic(D, over, 64, 96)
+
+
+@pytest.mark.parametrize("D", [1, 3, 4, 8, 12, 32])
+def test_loss_fused_with_the_upsample_on_an_odd_low_resolution_map(D):
+    """40x56 images: a 5x7 low-resolution map (35 cells per image, neither even nor a multiple of 4)."""
+    _check_fused_loss_equals_generic(D, {}, 40, 56)
+
+
+def _check_fused_loss_equals_generic(D, over, H, W):
+    B = 2
     h, w, P = H // 8, W // 8, H * W
     gen = torch.Generator().manual_seed(21)
     low = [(0.3 * torch.randn(B, h * w, D, generator=gen)).to(DEV) for _ in range(2)]

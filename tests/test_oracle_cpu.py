@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from oracle import loss_oracle as LO
+from oracle import well_conditioned as WC
 from oracle.resnet34_8s_oracle import GOLDEN_CPU_THREADS, seeded_oracle, process_network_output
 import pdc_b200
 from pdc_b200 import synthetic
@@ -200,3 +201,16 @@ def test_reprojection_oracle_against_ray_cast_ground_truth():
     ma = torch.randint(0, H * W, (40,), generator=torch.Generator().manual_seed(5))
     na, nb = LO.create_non_correspondences_flat(ma, (H, W), 7, mask, ru, rv)
     assert torch.equal(na, ma.repeat_interleave(7)) and bool((mask.view(-1)[nb] == 1).all())
+
+
+@pytest.mark.parametrize("case", WC.CASES, ids=WC.case_id)
+def test_well_conditioned_fixtures_have_their_certificate(case):
+    """Every input the whole-network fp64 gradient gate of the GPU suite may try (oracle/well_conditioned.py): the fp32 oracle's
+    parameter gradients lie within 1e-4 (relative, per tensor) of fp64 -- so a failure of that gate is the network's, not the
+    inputs'."""
+    D, B, groups, H, W, mode, seeds = case
+    for seed in seeds:
+        x, cot, oracle = WC.build(mode, D, B, H, W, seed, groups)
+        _, _, big, _, cert = WC.reference(oracle, mode, x, cot, groups)
+        assert cert < 1e-4, (seed, cert)
+        assert len(big) > 100          # of ~110 parameter tensors: only the cancelling fc.bias gradient is negligible
