@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define DDN_ABI_VERSION 2
+#define DDN_ABI_VERSION 3
 
 enum {
   DDN_OK = 0,
@@ -39,10 +39,6 @@ enum {
 };
 
 int ddn_abi_version(void);
-/* Data-parallel hosts: leave `n` SMs (0..64; default 0, or $DDN_RESERVED_SMS) free of the persistent tensor-core kernels so that a
- * concurrent collective (the NCCL all-reduce a ddn_grad_bucket_fn callback starts inside ddn_resnet34_8s_backward) has SMs to run on.
- * No reference counterpart: the reference is single-GPU (dense_correspondence/training/training.py:254-256). */
-int ddn_set_reserved_sms(int n);
 const char* ddn_last_error(void);
 
 /* ------------------------------------------------------------------------------------------

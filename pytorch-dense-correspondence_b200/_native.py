@@ -45,7 +45,6 @@ class WithinSceneCfg(ctypes.Structure):
 
 _SIGNATURES = {
     "ddn_abi_version": (i32, []),
-    "ddn_set_reserved_sms": (i32, [i32]),
     "ddn_last_error": (ctypes.c_char_p, []),
     "ddn_kernel_launch_count": (i64, []),
     "ddn_resnet34_8s_param_table": (i32, [i32, ctypes.POINTER(TensorEntry), i32]),
@@ -108,7 +107,7 @@ def _load():
         fn = getattr(lib, name)      # AttributeError here == header/library mismatch: fail loudly
         fn.restype = res
         fn.argtypes = args
-    if lib.ddn_abi_version() != 2:
+    if lib.ddn_abi_version() != 3:
         raise ImportError("libddn_b200.so ABI version mismatch")
     return lib
 

@@ -48,39 +48,44 @@ void set_error(const char* fmt, ...);
 // them (and, in the persistent tcgen05 kernels, overlaps barrier init / TMEM allocation with the predecessor's tail).
 // Rule: nothing written by an earlier kernel may be read before pdl_wait(), and EVERY thread of every kernel executes it
 // (a kernel that skipped it could finish before its predecessor and break the chain for its successor).
-// DDN_PDL=0 launches without the attribute (the instructions are then no-ops).
-bool pdl_enabled();
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_prologue() { pdl_trigger(); pdl_wait(); }
 
+// cluster_x > 1 groups the grid's CTAs along x into clusters of that size (the CTA pairs of the tcgen05 cta_group::2 kernels).
 template <typename... KArgs, typename... Args>
-static inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+static inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, unsigned cluster_x, dim3 block, size_t smem, cudaStream_t st,
+                                        Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  if (pdl_enabled()) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
+  cudaLaunchAttribute attr[2];
+  int n = 0;
+  if (cluster_x > 1) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = cluster_x; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = 1;
+    ++n;
   }
+  attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
+  cfg.attrs = attr; cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 #endif
 
-// Every kernel launch goes through this so gpu_launches is an honest count.
-#define DDN_LAUNCH(kernel, grid, block, smem, stream, ...)                                        \
-  do {                                                                                            \
-    DDN_CUDA(::ddn::launch_kernel(kernel, dim3(grid), dim3(block), (smem), (stream), __VA_ARGS__)); \
-    ::ddn::g_launches.fetch_add(1, std::memory_order_relaxed);                                    \
+// Every kernel launch goes through one of these so gpu_launches is an honest count.
+#define DDN_LAUNCH_CLUSTER(kernel, grid, cluster_x, block, smem, stream, ...)                                        \
+  do {                                                                                                               \
+    DDN_CUDA(::ddn::launch_kernel(kernel, dim3(grid), (unsigned)(cluster_x), dim3(block), (smem), (stream), __VA_ARGS__)); \
+    ::ddn::g_launches.fetch_add(1, std::memory_order_relaxed);                                                       \
   } while (0)
+#define DDN_LAUNCH(kernel, grid, block, smem, stream, ...) DDN_LAUNCH_CLUSTER(kernel, grid, 1, block, smem, stream, __VA_ARGS__)
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t a, size_t b) { return (a + b - 1) / b * b; }
 
 int num_sms();
-int tc_worker_sms();      // num_sms() minus the SMs reserved for a concurrent collective (ddn_set_reserved_sms)
 
 // Optional per-kernel-class timing with CUDA events on the launching stream (off by default; bench.py turns it on).
 enum ProfClass { PROF_CONV_FWD_SIMT = 0, PROF_CONV_DGRAD_SIMT, PROF_CONV_WGRAD_SIMT, PROF_CONV_FWD_TC, PROF_CONV_DGRAD_TC,

@@ -1658,10 +1658,9 @@ static int make_weight_map(CUtensorMap* m, const void* base, int rows, int K, in
   return 0;
 }
 
-static bool tc_halo_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_TC_HALO"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
+// layer1's 64 -> 64 3x3 convolutions, whose (output) map tiles by HALO_TH x HALO_TW, run on the halo-tile kernels
+static bool tc_halo_shape(int k, int cin, int cout, int stride, int dil, int H, int W) {
+  return k == 3 && cin == 64 && cout == 64 && stride == 1 && dil == 1 && H % HALO_TH == 0 && W % HALO_TW == 0;
 }
 
 template <int BN, int T, int NPROD>
@@ -1692,7 +1691,7 @@ int tc_wgrad_planes(TcPlanes x, TcPlanes dy, float* dw, int N, int H, int W, int
   const int taps = k * k;
   const int Ho = H / stride, Wo = W / stride;
   if (dw) DDN_TRY(launch_fill_zero(dwp, sizeof(float) * (size_t)taps * Cout * Cin, st));
-  if (tc_halo_enabled() && k == 3 && Cin == 64 && Cout == 64 && stride == 1 && dil == 1 && H % HALO_TH == 0 && W % HALO_TW == 0) {
+  if (tc_halo_shape(k, Cin, Cout, stride, dil, H, W)) {
     // layer1: one halo tile of X + one tile of dY per 8x16 pixels, two taps stacked per MMA (wgrad64_halo_kernel)
     TcWgradHaloParams hp;
     hp.dwp = dwp; hp.N = N; hp.H = H; hp.W = W; hp.tiles_h = H / HALO_TH; hp.tiles_w = W / HALO_TW; hp.n_tiles = N * hp.tiles_h * hp.tiles_w;
@@ -1703,7 +1702,7 @@ int tc_wgrad_planes(TcPlanes x, TcPlanes dy, float* dw, int N, int H, int W, int
     DDN_TRY(make_act_map_hw(&md_lo, want_lo ? dy.lo : dy.hi, N, H, W, 64, HALO_TH, HALO_TW));
     const int nsplit = want_lo ? 2 : 1;
     const size_t smem = (size_t)2 * nsplit * (WGH_X_SLOT + WGH_DY_BYTES) + 1024;
-    const int grid = std::min(hp.n_tiles, tc_worker_sms());
+    const int grid = std::min(hp.n_tiles, num_sms());
     {
       ProfScope ps(PROF_CONV_WGRAD_TC, 2.0 * N * H * W * 64.0 * 9 * 64, st);
       if (want_lo) {
@@ -1734,7 +1733,7 @@ int tc_wgrad_planes(TcPlanes x, TcPlanes dy, float* dw, int N, int H, int W, int
   const int total_kb = N * p.tiles_h * p.tiles_w;
   const int ctas_xy = (Cin / bn) * (k == 3 ? 3 : 1) * (int)ceil_div(Cout, 128);
   // split-K so that the grid is (just under) a whole number of waves: 1 CTA per SM resident, no ragged tail wave
-  const int sms = tc_worker_sms();
+  const int sms = num_sms();
   int waves = ctas_xy > sms ? 1 : (total_kb >= 64 * (sms / ctas_xy) ? 2 : 1);
   int splits = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)waves * sms / ctas_xy, ceil_div(total_kb, 4)));
   p.kb_per_split = (int)ceil_div(total_kb, splits);
@@ -1770,11 +1769,6 @@ int tc_unpack_wgrads(const TcUnpackEntry* entries, int n, const float* dwp_base,
 }
 
 bool tc_available() { return true; }
-bool tc_folded_epilogue_supported() {      // DDN_FOLD_BN=0: keep the separate eval-mode BN pass (A/B measurements)
-  static int fold = -1;
-  if (fold < 0) { const char* e = getenv("DDN_FOLD_BN"); fold = (e && e[0] == '0') ? 0 : 1; }
-  return fold != 0;
-}
 
 // forward / weight-gradient coverage: 3x3 (pad == dil) or 1x1 (pad 0), stride 1 -- or stride 2 with dil 1 on even sizes
 bool tc_conv_supported(int Cin, int Cout, int k, int stride, int pad, int dil, int H, int W) {
@@ -1821,18 +1815,6 @@ int tc_stem_patches(const float* x_nchw, __nv_bfloat16* hi, __nv_bfloat16* lo, i
   return 0;
 }
 
-// DDN_TC_PAIR=0: never use the CTA-pair kernel (A/B measurements); DDN_TC_TAIL=0: no N-split of the tail wave
-static bool tc_pair_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_TC_PAIR"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-static bool tc_tail_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_TC_TAIL"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-
 template <int BLOCK_N, int NPROD, bool PAIR>
 static int launch_conv_tc(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const CUtensorMap& b_hi, const CUtensorMap& b_lo,
                           const CUtensorMap& bt_hi, const CUtensorMap& bt_lo, const TcConvParams& p, int workers, cudaStream_t st) {
@@ -1846,26 +1828,8 @@ static int launch_conv_tc(const CUtensorMap& a_hi, const CUtensorMap& a_lo, cons
     DDN_CUDA(cudaFuncSetAttribute(conv_tc_kernel<BLOCK_N, NPROD, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(PAIR ? 2 * workers : workers));
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int n_attr = 0;
-  if (PAIR) {
-    attr[n_attr].id = cudaLaunchAttributeClusterDimension;
-    attr[n_attr].val.clusterDim.x = 2; attr[n_attr].val.clusterDim.y = 1; attr[n_attr].val.clusterDim.z = 1;
-    ++n_attr;
-  }
-  if (pdl_enabled()) {
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
-    ++n_attr;
-  }
-  cfg.attrs = attr; cfg.numAttrs = n_attr;
-  DDN_CUDA(cudaLaunchKernelEx(&cfg, conv_tc_kernel<BLOCK_N, NPROD, PAIR>, a_hi, a_lo, b_hi, b_lo, bt_hi, bt_lo, p));
-  g_launches.fetch_add(1, std::memory_order_relaxed);
+  DDN_LAUNCH_CLUSTER((conv_tc_kernel<BLOCK_N, NPROD, PAIR>), PAIR ? 2 * workers : workers, PAIR ? 2 : 1, TC_THREADS, smem, st,
+                     a_hi, a_lo, b_hi, b_lo, bt_hi, bt_lo, p);
   return 0;
 }
 
@@ -1879,7 +1843,7 @@ static int launch_conv64_halo(const CUtensorMap& a_hi, const CUtensorMap& a_lo, 
     DDN_CUDA(cudaFuncSetAttribute(conv64_halo_kernel<NPROD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
-  const int grid = std::min(p.n_tiles, tc_worker_sms());
+  const int grid = std::min(p.n_tiles, num_sms());
   DDN_LAUNCH((conv64_halo_kernel<NPROD>), grid, TC_THREADS, smem, st, a_hi, a_lo, b_hi, b_lo, p);
   return 0;
 }
@@ -1915,7 +1879,7 @@ int tc_conv_planes(TcPlanes in, const float* w_oihw, const TcPlanes* wpk, float*
     DDN_LAUNCH(pack_weights_tc_kernel, wblocks, 256, 0, st, w_oihw, ph, pl, Cout, Cin, k, dgrad, want_lo);
     b_hi = ph; b_lo = pl;
   }
-  if (tc_halo_enabled() && k == 3 && gin == 64 && gout == 64 && stride == 1 && dil == 1 && Ho % HALO_TH == 0 && Wo % HALO_TW == 0) {
+  if (tc_halo_shape(k, gin, gout, stride, dil, Ho, Wo)) {
     // 64 -> 64 channels (layer1): resident weights + one halo tile per 8x16 output pixels (conv64_halo_kernel)
     TcHaloParams hp;
     memset(&hp, 0, sizeof(hp));
@@ -1948,12 +1912,10 @@ int tc_conv_planes(TcPlanes in, const float* w_oihw, const TcPlanes* wpk, float*
     ProfScope ps(dgrad ? PROF_CONV_DGRAD_TC : PROF_CONV_FWD_TC, fl, st);
     return want_lo ? launch_conv64_halo<3>(ma_hi, ma_lo, mb_hi, mb_lo, hp, st) : launch_conv64_halo<1>(ma_hi, ma_lo, mb_hi, mb_lo, hp, st);
   }
-  // CTA pairs for Cout % 256 == 0 (256 x 256 tiles).  DDN_TC_PAIR128=1 also pairs Cout = 128 (layer2, 256 x 128 tiles: each CTA
-  // stages half of the weight rows, 25 % less L2 -> SM traffic per pixel on a layer that runs at that throughput cap): parity-green,
-  // but 279.7 vs 279.3 pairs/s in a 3 x 2 one-call A/B -- noise -- so the single-CTA 128 x 128 tiles stay the default.
-  static const bool pair128 = [] { const char* e = getenv("DDN_TC_PAIR128"); return e && e[0] == '1'; }();
-  const bool pair = tc_pair_enabled() && (gout % 256 == 0 || (pair128 && gout == 128));
-  const int block_n = pair ? (gout % 256 == 0 ? 256 : 128) : gout % 128 == 0 ? 128 : 64;
+  // CTA pairs (256 x 256 tiles) for Cout % 256 == 0.  Pairing Cout = 128 as 256 x 128 tiles measured no faster than single CTAs
+  // (DESIGN.md §8).
+  const bool pair = gout % 256 == 0;
+  const int block_n = pair ? 256 : gout % 128 == 0 ? 128 : 64;
   TcConvParams p;
   memset(&p, 0, sizeof(p));
   p.out = out; p.addend = addend; p.N = N; p.H = Ho; p.W = Wo; p.Cin = gin; p.Cout = gout; p.taps_w = k; p.dil = dil;
@@ -1963,12 +1925,12 @@ int tc_conv_planes(TcPlanes in, const float* w_oihw, const TcPlanes* wpk, float*
   p.n_co = gout / block_n;
   const int subs_per_tile = pair ? 4 : 2;
   const int tiles = (int)ceil_div(p.n_sub, subs_per_tile) * p.n_co;
-  const int workers_max = pair ? tc_worker_sms() / 2 : tc_worker_sms();
+  const int workers_max = pair ? num_sms() / 2 : num_sms();
   // the tiles of the last, partial wave are cut along N so that the tail costs a fraction of a tile time
   const int rem = tiles % workers_max;
   const int min_width = pair ? 64 : 32;
   int split = 1;
-  if (rem && tc_tail_enabled())
+  if (rem)
     while (split * 2 <= 8 && block_n / (split * 2) >= min_width && rem * split * 2 <= workers_max) split *= 2;
   p.full_items = tiles - rem; p.tail_split = split; p.total_items = p.full_items + rem * split;
   if (split == 1) { p.full_items = tiles; p.total_items = tiles; }
@@ -2005,8 +1967,7 @@ int tc_conv_planes(TcPlanes in, const float* w_oihw, const TcPlanes* wpk, float*
 #define CONV_TC(BN, PR)                                                                                                       \
   (want_lo ? launch_conv_tc<BN, 3, PR>(ma_hi, ma_lo, mb_hi, mb_lo, mt_hi, mt_lo, p, workers, st)                               \
            : launch_conv_tc<BN, 1, PR>(ma_hi, ma_lo, mb_hi, mb_lo, mt_hi, mt_lo, p, workers, st))
-  if (pair && block_n == 256) return CONV_TC(256, true);
-  if (pair) return CONV_TC(128, true);
+  if (pair) return CONV_TC(256, true);
   if (block_n == 128) return CONV_TC(128, false);
   return CONV_TC(64, false);
 #undef CONV_TC

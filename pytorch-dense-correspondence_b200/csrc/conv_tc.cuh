@@ -11,7 +11,6 @@ struct TcPlanes { const __nv_bfloat16* hi; const __nv_bfloat16* lo; };   // x ~=
 // the conv (scale = gamma / sqrt(running_var + eps), shift = beta - running_mean * scale) -- written as fp32 (`out`, may be
 // null) and / or as the bf16 hi/lo operand planes of the next conv.
 struct TcFoldedEpilogue { const float* scale; const float* shift; int relu; __nv_bfloat16* out_hi; __nv_bfloat16* out_lo; };
-bool tc_folded_epilogue_supported();
 
 // Data-gradient epilogue that also produces the column sums of the BatchNorm backward consuming the gradient it writes:
 // out = dY of y = relu?(bn(raw) [+ residual]); g = out * (y > 0) with the mask taken from the bf16 hi plane of y (`y_hi`, blocks

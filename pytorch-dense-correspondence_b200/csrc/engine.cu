@@ -24,34 +24,6 @@ void set_error(const char* fmt, ...) {
   va_end(ap);
 }
 
-bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_PDL"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v != 0;
-}
-
-// SMs left free by the persistent tcgen05 kernels (one CTA per SM, no room for a second): while a data-parallel host has a gradient
-// all-reduce in flight, NCCL's CTAs need somewhere to run -- without the reservation they take SMs between two of our launches and
-// the next persistent kernel runs a whole extra wave for the CTAs that found no SM.  Set by ddn_set_reserved_sms (DDN_RESERVED_SMS).
-static std::atomic<int> g_reserved_sms{-1};
-// ... and the same for a WINDOW only: from the first gradient bucket a backward hands to its host (whose all-reduce then runs
-// concurrently) to the end of that backward (DDN_OVERLAP_RESERVED_SMS = n; the host then caps NCCL at n CTAs).  Measured on
-// 2 x B200 in one call (profiles/r2_reserved_sms_ab.md): n = 0 538, n = 4 545, n = 8 537, n = 16 528 pairs/s -- inside the +-1 %
-// run-to-run noise, so the default is 0 (no reservation, NCCL's own CTA count).
-static std::atomic<int> g_window_reserved{0};
-static int overlap_window_sms() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_OVERLAP_RESERVED_SMS"); v = e ? atoi(e) : 0; if (v < 0 || v > 64) v = 0; }
-  return v;
-}
-int tc_worker_sms() {
-  int r = g_reserved_sms.load(std::memory_order_relaxed);
-  if (r < 0) { const char* e = getenv("DDN_RESERVED_SMS"); r = e ? atoi(e) : 0; if (r < 0) r = 0; g_reserved_sms.store(r); }
-  r = std::max(r, g_window_reserved.load(std::memory_order_relaxed));
-  const int n = num_sms();
-  return r >= n - 8 ? 8 : n - r;
-}
-
 int num_sms() {
   static int n = 0;
   if (n == 0) {
@@ -422,7 +394,7 @@ static int net_forward(const Ctx& c, const float* x, float* y, float* low_nhwc) 
   const NetSpec& s = *c.s; const Plan& p = *c.p;
   const int B = p.B, G = c.G;
   const bool want_lo = p.precision == DDN_PRECISION_BF16X3;
-  const bool fold = c.mode == DDN_MODE_INFER && p.tc && tc_folded_epilogue_supported();
+  const bool fold = c.mode == DDN_MODE_INFER && p.tc;
   DDN_CUDA(cudaMemsetAsync(c.ws + p.acc, 0, bn_accum_bytes(512), c.st));     // the workspace arrives uninitialised
   if (p.tc) DDN_TRY(ensure_packs(c));
   if (!c.training() && !fold) DDN_TRY(fill_eval_stats(c));
@@ -571,15 +543,9 @@ static int bn_backward_for(const Ctx& c, const BnSpec& bs, const ConvBufs& cb, c
 }
 
 // Column sums of BatchNorm `bs` (y = relu(bn(raw) [+ residual])) computed by the epilogue of the tensor-core data gradient that
-// produces its dY (conv_tc.cuh TcBwdStats) instead of a separate pass over dY and raw.  DDN_FUSE_BWD_STATS_MINC (default 64 = every
-// layer) keeps the separate pass for layers narrower than that many channels (A/B switch).
-static int fuse_bwd_stats_min_c() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DDN_FUSE_BWD_STATS_MINC"); v = e ? atoi(e) : 64; if (v < 0) v = 0; }
-  return v;
-}
+// produces its dY (conv_tc.cuh TcBwdStats) instead of a separate pass over dY and raw.
 static bool bwd_stats_for(const Ctx& c, const BnSpec& bs, const ConvBufs& cb, const __nv_bfloat16* y_hi, int slot, TcBwdStats* out) {
-  if (!c.p->tc || bs.C < fuse_bwd_stats_min_c()) return false;
+  if (!c.p->tc) return false;
   memset(out, 0, sizeof(*out));
   out->raw = c.f(cb.raw); out->y_hi = y_hi; out->mean = c.mean(cb.stats); out->invstd = c.invstd(cb.stats, bs.C);
   out->gamma = c.params + bs.g_off; out->beta = c.params + bs.b_off; out->relu = 1;
@@ -614,14 +580,10 @@ static int net_backward(const Ctx& c, const float* dy, const float* dlow_nhwc, d
   };
   int64_t bucket_end = s.n_params;
   int bucket_id = 0;
-  struct WindowGuard { ~WindowGuard() { g_window_reserved.store(0, std::memory_order_relaxed); } } window_guard;
   auto close_bucket = [&](int64_t begin) -> int {
     if (!pending.empty()) DDN_TRY(tc_unpack_wgrads(pending.data(), (int)pending.size(), c.f(p.dwp_all), c.grads, c.st));
     pending.clear();
-    if (on_bucket) {
-      on_bucket(user, bucket_id, begin, bucket_end - begin);
-      g_window_reserved.store(overlap_window_sms(), std::memory_order_relaxed);     // a collective is in flight from here on
-    }
+    if (on_bucket) on_bucket(user, bucket_id, begin, bucket_end - begin);
     ++bucket_id; bucket_end = begin;
     return 0;
   };
@@ -701,11 +663,6 @@ static int net_backward(const Ctx& c, const float* dy, const float* dlow_nhwc, d
 using namespace ddn;
 
 extern "C" int ddn_abi_version(void) { return DDN_ABI_VERSION; }
-extern "C" int ddn_set_reserved_sms(int n) {
-  DDN_CHECK_ARG(n >= 0 && n <= 64, "reserved SM count must be in [0, 64]");
-  g_reserved_sms.store(n);
-  return 0;
-}
 extern "C" const char* ddn_last_error(void) { return g_err; }
 extern "C" int64_t ddn_kernel_launch_count(void) { return g_launches.load(); }
 

@@ -464,8 +464,8 @@ extern "C" int ddn_contrastive_terms_forward_lowres(const float* low_a, const fl
   DDN_CHECK_ARG(sums && counts && h >= 1 && w >= 1 && H >= h && W >= w && (int64_t)H * W < (1LL << 31), "bad low-resolution geometry / null outputs");
   DDN_CHECK_ARG(lowres_aligned(D, low_a, low_b), "low-resolution maps must be 16-byte aligned when D is a multiple of 4");
   const int lpp = (D == 8 || D == 16 || D == 32) ? D / 4 : 1;
-  // 4 pairs per lane group; 8 (DDN_LOSS_FWD_ITEMS=8) halves the atomics again but costs occupancy: 17.4 -> 18.7-20.9 us at C3
-  static const int items = [] { const char* e = getenv("DDN_LOSS_FWD_ITEMS"); return (e && atoi(e) == 8) ? 8 : 4; }();
+  // 4 pairs per lane group; 8 halves the atomics again but costs occupancy: 17.4 -> 18.7-20.9 us at C3 (DESIGN.md §8)
+  constexpr int items = 4;
   DevTerms T;
   DDN_TRY(build_terms_lr(terms_host, n_terms, &T, lpp > 1 ? LR_THREADS / lpp * items : LR_THREADS));
   cudaStream_t st = (cudaStream_t)stream;
@@ -479,11 +479,7 @@ extern "C" int ddn_contrastive_terms_forward_lowres(const float* low_a, const fl
   ProfScope ps(PROF_LOSS_FWD, pairs * (16.0 + 8.0 * D), st);
   const float sh = ac_scale(h, H), sw = ac_scale(w, W);
 #define FWD(DT) DDN_LAUNCH(loss_lowres_fwd_kernel<DT>, grid, LR_THREADS, 0, st, low_a, low_b, h, w, H, W, D, sh, sw, T, sums, cnt)
-#define FWDQ(L)                                                                                                                              \
-  do {                                                                                                                                       \
-    if (items == 4) DDN_LAUNCH((loss_lowres_fwd_quad_kernel<L, 4>), grid, LR_THREADS, 0, st, low_a, low_b, h, w, H, W, sh, sw, T, sums, cnt); \
-    else DDN_LAUNCH((loss_lowres_fwd_quad_kernel<L, 8>), grid, LR_THREADS, 0, st, low_a, low_b, h, w, H, W, sh, sw, T, sums, cnt);            \
-  } while (0)
+#define FWDQ(L) DDN_LAUNCH((loss_lowres_fwd_quad_kernel<L, items>), grid, LR_THREADS, 0, st, low_a, low_b, h, w, H, W, sh, sw, T, sums, cnt)
   switch (D) {
     case 3: FWD(3); break;
     case 4: FWD(4); break;

@@ -24,12 +24,6 @@ def init_from_env(backend=None):
             backend = "nccl" if torch.cuda.is_available() else "gloo"
         if backend == "nccl":
             torch.cuda.set_device(local_rank)
-            # Experiments, both off by default (profiles/r2_reserved_sms_ab.md): DDN_OVERLAP_RESERVED_SMS=n keeps n SMs free of the
-            # persistent kernels from the first gradient bucket to the end of the backward, DDN_RESERVED_SMS=n for the whole step;
-            # NCCL is then capped at n CTAs so that it fits there.
-            cap = max(int(os.environ.get("DDN_OVERLAP_RESERVED_SMS", "0")), int(os.environ.get("DDN_RESERVED_SMS", "0")))
-            if cap > 0:
-                os.environ.setdefault("NCCL_MAX_CTAS", str(cap))
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         os.environ.setdefault("MASTER_PORT", "29500")
         dist.init_process_group(backend=backend, rank=rank, world_size=world)
@@ -108,16 +102,8 @@ class GradientAllReducer(object):
         self.module = module
         if module is not None and overlap and dist.is_initialized() and dist.get_world_size(group) > 1:
             module._bucket_hook = self
-            self._reserve_sms(int(os.environ.get("DDN_RESERVED_SMS", "0")))
         elif module is not None:
             module._bucket_hook = None
-
-    @staticmethod
-    def _reserve_sms(n):
-        """SMs the persistent tensor-core kernels leave free for NCCL while an all-reduce overlaps the backward."""
-        if torch.cuda.is_available():
-            from . import _native as N
-            N.check(N.lib.ddn_set_reserved_sms(int(n)))
 
     # ---- overlapped path: called by resnet_dilated._Backbone.backward
     def cotangent_scale(self):
@@ -143,7 +129,6 @@ class GradientAllReducer(object):
     def detach(self):
         if self.module is not None and getattr(self.module, "_bucket_hook", None) is self:
             self.module._bucket_hook = None
-            self._reserve_sms(0)
 
     # ---- explicit path
     def __call__(self):

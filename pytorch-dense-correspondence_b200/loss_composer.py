@@ -10,8 +10,6 @@ Batch extension (the reference is batch-1 only, training.py:314-323): descriptor
 ``[B, W*H, D]`` with ``[B, n]`` index tensors; the loss is then the mean over the B pairs of the reference's
 per-pair loss (SURVEY.md 8a).
 """
-import os
-
 import torch
 
 from . import _native as N
@@ -21,10 +19,8 @@ from .resnet_dilated import lowres_of
 
 def _fused_lowres(image_a_pred, image_b_pred, image_width):
     """When both descriptor images are untouched outputs of Resnet34_8s (they carry the low-resolution map they were upsampled
-    from), the loss is evaluated THROUGH the upsample: (low_a, low_b, (h, w, H, W)), else None.  DDN_FUSED_UPSAMPLE_LOSS=0
-    forces the generic gather from the full-resolution images (A/B measurements, tests)."""
-    if os.environ.get("DDN_FUSED_UPSAMPLE_LOSS", "1") == "0":
-        return None
+    from), the loss is evaluated THROUGH the upsample: (low_a, low_b, (h, w, H, W)), else None (the generic gather from the
+    full-resolution images)."""
     ta, tb = lowres_of(image_a_pred), lowres_of(image_b_pred)
     if ta is None or tb is None or ta[1:3] != tb[1:3] or ta[2] != image_width or ta[0].shape != tb[0].shape:
         return None

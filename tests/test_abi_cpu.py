@@ -27,7 +27,7 @@ def test_header_symbols_exported_and_bound():
     for n in names:
         assert hasattr(lib, n), "declared in ddn_b200.h but not exported: " + n
     assert set(names) == set(N.EXPORTED_SYMBOLS), set(names) ^ set(N.EXPORTED_SYMBOLS)
-    assert N.lib.ddn_abi_version() == 2
+    assert N.lib.ddn_abi_version() == 3
 
 
 @pytest.mark.parametrize("D", [3, 8, 16])
@@ -73,9 +73,6 @@ def test_workspace_and_argument_checks():
     assert N.lib.ddn_conv2d_workspace_bytes(1, 60, 80, 64, 64, 3, 1, 1, 1, 0) >= 3 * 9 * 64 * 64 * 4
     assert N.lib.ddn_batchnorm_workspace_bytes(4800, 6) == 0 and N.lib.ddn_batchnorm_workspace_bytes(4800, 512) > 0
     assert N.launch_count() == before
-    # SM reservation for a concurrent collective: a host-side setting with a range check (INTEGRATION.md A, data parallel)
-    assert N.lib.ddn_set_reserved_sms(8) == 0 and N.lib.ddn_set_reserved_sms(0) == 0
-    assert N.lib.ddn_set_reserved_sms(-1) == -1 and N.lib.ddn_set_reserved_sms(1000) == -1
     with pytest.raises(N.DdnError):
         N.check(-1)
 

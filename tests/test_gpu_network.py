@@ -539,17 +539,16 @@ def test_full_size_forward_other_descriptor_dimensions(D):
     assert rel(ye, ye_o) < 1e-3 and relmax(ye, ye_o) < 1e-3
 
 
-def test_step_with_fused_upsample_loss_equals_generic_path(monkeypatch):
+def test_step_with_fused_upsample_loss_equals_generic_path():
     """forward_pair + get_loss + backward with the loss fused into the upsample (default) vs the generic full-resolution gather
-    (DDN_FUSED_UPSAMPLE_LOSS=0): same loss, same parameter gradients (fc tightly; all within the train-mode noise floor)."""
+    (a clone drops the low-resolution tag): same loss, same parameter gradients (fc tightly; all within the train-mode noise floor)."""
     tc_or_skip("bf16x3")
     D, B, H, W = 3, 2, 64, 96
     data = synthetic.make_pair_batch(B, H, W, 40, 120, 120, 0, seed=31)
     d = {k: (v.to(DEV) if v is not None else None) for k, v in data.items()}
     blind = loss_composer.empty_tensor().to(DEV)
     outs = {}
-    for fused in ("1", "0"):
-        monkeypatch.setenv("DDN_FUSED_UPSAMPLE_LOSS", fused)
+    for fused in (True, False):
         dcn = pdc_b200.DenseCorrespondenceNetwork.from_config({"descriptor_dimension": D, "image_width": W, "image_height": H},
                                                               load_stored_params=False)
         dcn.fcn.load_state_dict(seeded_oracle(D=D, seed=0).state_dict())
@@ -558,11 +557,14 @@ def test_step_with_fused_upsample_loss_equals_generic_path(monkeypatch):
         a, b = dcn.forward_pair(d["img_a"], d["img_b"])
         pa, pb = dcn.process_network_output(a, B), dcn.process_network_output(b, B)
         assert (pdc_b200.resnet_dilated.lowres_of(pa) is not None)
+        if not fused:
+            pa, pb = pa.clone(), pb.clone()
+            assert pdc_b200.resnet_dilated.lowres_of(pa) is None and pdc_b200.resnet_dilated.lowres_of(pb) is None
         five = loss_composer.get_loss(pcl, torch.zeros(B, dtype=torch.int64), pa, pb, d["matches_a"], d["matches_b"], d["masked_a"],
                                       d["masked_b"], d["background_a"], d["background_b"], blind, blind)
         five[0].backward()
         outs[fused] = ([float(t) for t in five], {k: p.grad.detach().clone() for k, p in dcn.fcn.named_parameters()})
-    (f1, g1), (f0, g0) = outs["1"], outs["0"]
+    (f1, g1), (f0, g0) = outs[True], outs[False]
     for x, y in zip(f1, f0):
         assert abs(x - y) <= 2e-6 * max(1.0, abs(y))
     assert rel(g1["resnet34_8s.fc.weight"], g0["resnet34_8s.fc.weight"]) < 1e-4
@@ -605,9 +607,9 @@ def _hard_negative_bounds(A, Bm, ia, ib, margin):
 
 @pytest.mark.parametrize("api", ["two_calls", "forward_pair"])
 @pytest.mark.parametrize("D,B,H,W", LOSS_SHAPES)
-def test_fused_loss_step_at_the_shape_matrix(monkeypatch, api, D, B, H, W):
+def test_fused_loss_step_at_the_shape_matrix(api, D, B, H, W):
     """A training step (forward A / B, get_loss with all four terms, backward) at the shapes and descriptor sizes of
-    oracle/well_conditioned.py: the loss fused with the upsample (default) equals the generic gather (DDN_FUSED_UPSAMPLE_LOSS=0)
+    oracle/well_conditioned.py: the loss fused with the upsample (default) equals the generic gather (on clones, which drop the tag)
     -- five outputs, hard-negative counts, parameter gradients -- and the fused loss equals the float64 restatement
     LO.np_within_scene_loss evaluated on the network's own descriptors.  Low-resolution maps with h*w odd or not a multiple of 4
     (40x48: 30 cells, 72x40: 45) put forward_pair's second half at an offset that is not 16-byte aligned."""
@@ -616,8 +618,7 @@ def test_fused_loss_step_at_the_shape_matrix(monkeypatch, api, D, B, H, W):
     d = {k: v.to(DEV) for k, v in data.items()}
     cfg = dict(LO.DEFAULT_LOSS_CONFIG)
     outs = {}
-    for fused in ("1", "0"):
-        monkeypatch.setenv("DDN_FUSED_UPSAMPLE_LOSS", fused)
+    for fused in (True, False):
         dcn = pdc_b200.DenseCorrespondenceNetwork.from_config({"descriptor_dimension": D, "image_width": W, "image_height": H},
                                                               load_stored_params=False)
         dcn.fcn.load_state_dict(seeded_oracle(D=D, seed=0).state_dict())
@@ -630,12 +631,15 @@ def test_fused_loss_step_at_the_shape_matrix(monkeypatch, api, D, B, H, W):
             a, b = dcn.forward(d["img_a"]), dcn.forward(d["img_b"])
         pa, pb = dcn.process_network_output(a, B), dcn.process_network_output(b, B)
         assert pdc_b200.resnet_dilated.lowres_of(pa) is not None and pdc_b200.resnet_dilated.lowres_of(pb) is not None
+        if not fused:
+            pa, pb = pa.clone(), pb.clone()
+            assert pdc_b200.resnet_dilated.lowres_of(pa) is None and pdc_b200.resnet_dilated.lowres_of(pb) is None
         five = loss_composer.get_loss(pcl, torch.zeros(B, dtype=torch.int64), pa, pb, d["matches_a"], d["matches_b"], d["masked_a"],
                                       d["masked_b"], d["background_a"], d["background_b"], d["blind_a"], d["blind_b"])
         five[0].backward()
         outs[fused] = ([float(t) for t in five], pcl.debug_data["num_hard_negatives_device"].cpu(),
                        {k: p.grad.detach().clone() for k, p in dcn.fcn.named_parameters()}, pa.detach().cpu(), pb.detach().cpu())
-    (f1, c1, g1, pa1, pb1), (f0, c0, g0, _, _) = outs["1"], outs["0"]
+    (f1, c1, g1, pa1, pb1), (f0, c0, g0, _, _) = outs[True], outs[False]
     assert torch.equal(c1, c0)
     for x, y in zip(f1, f0):
         assert abs(x - y) <= 2e-6 * max(1.0, abs(y)), (f1, f0)
